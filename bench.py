@@ -14,10 +14,12 @@ the per-candidate FP64 error sums are all-reduced (NCCL), so N ranks calibrate o
                                                             3 ViT-B W4A4 / 512 images in total (strong scaling),
                                                             4 DeiT-B W4A4 / 1024 in total (headline), 5 Swin-B W6A6 / 1024
   With --gpus 8 and the default config the line also carries a `headline` record: one calibration of config 4.
+  python bench.py --dump-outputs DIR [...]                  also write the calibrated model of the last timed step
+                                                            as DIR/<state_dict key>.npy (see dump_outputs)
 
 Prints ONE JSON line (rank 0).  `value` = candidate scorings per second with the images resident in HBM;
 `e2e` = the same through the public API starting from pinned host images (H2D inside the timed region) and ending
-with the calibrated quantizer parameters read back to the host.
+with the calibrated quantizer parameters read back to the host.  Both legs run --steps timed steps.
 """
 import argparse
 import copy
@@ -30,6 +32,7 @@ import sys
 import tempfile
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -77,7 +80,13 @@ def parse():
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-parity', action='store_true', help='skip the free-running parity / gpu_reference checker leg')
     ap.add_argument('--no-headline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the calibrated model of the last timed step as DIR/<state_dict key>.npy')
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs needs --impl ours: the reference arm times a sample of sweeps, not a calibration')
     world = int(os.environ.get('WORLD_SIZE', '1'))
     model, bits, images, scaling = CONFIGS[a.config or 2]
     a.scaling = scaling if a.images_per_gpu is None else 'weak'
@@ -316,6 +325,31 @@ def quant_params_to_host(model):
     return out, nbytes
 
 
+DUMP_SAMPLE = 1 << 16
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(model, out_dir):
+    """Writes the calibrated model's state_dict -- what a caller of the timed calibration receives, and what
+    test_quant.py saves as the checkpoint -- as out_dir/<key>.npy: float32 tensors as float32, every other dtype as
+    float64 (exact for the int64 base indices and the bool flags).  A tensor of more than DUMP_SAMPLE elements is
+    written flattened, as its elements at DUMP_SAMPLE fixed seeded positions (sorted), so two builds of the project
+    compare position for position; DeiT-S comes to about 14 MB instead of 88 MB."""
+    arrays = {}
+    for k, v in model.state_dict().items():
+        v = v.detach()
+        if v.numel() > DUMP_SAMPLE:
+            pos = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            v = v.reshape(-1)[pos.to(v.device)]
+        arrays[k] = v.to(torch.float32 if v.dtype == torch.float32 else torch.float64).cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError(f'--dump-outputs: {total} bytes exceed the {DUMP_LIMIT} byte limit')
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + '.npy'), a)
+
+
 def run_ours(args):
     import torch.distributed as dist
     from adalog_b200 import _lib, ops
@@ -391,11 +425,13 @@ def run_ours(args):
     gemm_launches = sum(v[2] for v in gemm_split.values()) + sum(v[2] for v in lin_split.values())
     launches = _lib.LAUNCHES['count']
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:      # every rank calibrates to the same parameters (errors are all-reduced)
+        dump_outputs(model, args.dump_outputs)
 
     e2e_ms, d2h = None, 0
     if not args.no_e2e:
         e_times, d2h = [], 0
-        for _ in range(max(1, min(args.steps, 2))):
+        for _ in range(args.steps):
             ms, wall, d2h, _ = one_step(True)
             e_times.append(ms)
         e2e_ms = statistics.mean(e_times)

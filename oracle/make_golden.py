@@ -347,11 +347,35 @@ def run_model(name, model_name, bits, n_img=8, bs=4, img=32):
             m.reparam_bias()
     with torch.no_grad():
         logits_final = model(images).clone()
-    evals = [dict(digest=sims_digest(e['sims']), shape=tuple(e['sims'].shape), k=e['k'], dim=e['dim'], idx=e['idx'].to(torch.int16))
+    evals = [dict(digest=sims_digest(e['sims']), shape=tuple(e['sims'].shape), k=e['k'], dim=e['dim'], idx=e['idx'])
              for e in tap.evals]
-    save(name, dict(kind='model', model=model_name, bits=bits, n_img=n_img, bs=bs, init_state=init_state, images=images,
-                    order=order, fp_logits=fp_logits, evals=evals, state_calib=state_calib, logits=logits,
-                    state_final=sd(model), logits_final=logits_final, memory=ref_shim._Props.total_memory // 2))
+    save(name, pack_model_golden(dict(
+        kind='model', model=model_name, bits=bits, n_img=n_img, bs=bs, init_state=init_state, images=images, order=order,
+        fp_logits=fp_logits, evals=evals, state_calib=state_calib, logits=logits, state_final=sd(model),
+        logits_final=logits_final, memory=ref_shim._Props.total_memory // 2)))
+
+
+def pack_model_golden(g):
+    """Keeps a model golden under 1 MB without dropping any value: every evaluation's top-k indices (candidate numbers,
+    0..127) become uint8 views of one shared storage, and a state tensor equal to the one before it in init_state ->
+    state_calib -> state_final is stored once.  torch.save writes shared storages once; the tests read the indices
+    through .to(torch.int64)."""
+    flat = torch.cat([e['idx'].reshape(-1) for e in g['evals']])
+    assert int(flat.min()) >= 0 and int(flat.max()) < 256
+    flat = flat.to(torch.uint8)
+    o = 0
+    for e in g['evals']:
+        n = e['idx'].numel()
+        e['idx'] = flat[o:o + n].view(e['idx'].shape)
+        o += n
+    prev = g['init_state']
+    for key in ('state_calib', 'state_final'):
+        st = g[key]
+        for k, v in st.items():
+            if k in prev and prev[k].dtype == v.dtype and prev[k].shape == v.shape and torch.equal(prev[k], v):
+                st[k] = prev[k]
+        prev = st
+    return g
 
 
 def main_models():
