@@ -24,7 +24,6 @@
 #include "quant_device.cuh"
 #include "../../include/adalog_b200.h"
 #include <type_traits>
-#include <stdlib.h>
 
 
 namespace adalog {
@@ -59,7 +58,7 @@ struct FArgs {
   const float* cs; const float* cz; long long pstride, gstride, g_div, g_mod;
   const long long* cq; const float* mtab;
   int P, nl;
-  int KB, N, BN, U, UG, cpg, nst, nacc, acc_cols, epi_warps, dbg;
+  int KB, N, BN, U, UG, cpg, nst, nacc, acc_cols, epi_warps;
   long long brpg, g_base, u_base;
   const float* y; long long ldy;
   const float* rs; long long rs_div, rs_mod;
@@ -270,7 +269,6 @@ fused_cand_gemm_err_kernel(const __grid_constant__ CUtensorMap tmB, const FArgs 
       for (int sl = eg; sl < nslab; sl += 2 * G, l0 += 64) {
         tmem_ld_wait();
         if (sl + G < nslab) tmem_ld32(tbase + (sl + G) * 32, db);
-        if (a.dbg & 2) { acc4[0] += __uint_as_float(da[0]); continue; }
         consume(da, l0, a.N - sl * 32);
         if (sl + G < nslab) {
           tmem_ld_wait();
@@ -317,7 +315,7 @@ fused_cand_gemm_err_kernel(const __grid_constant__ CUtensorMap tmB, const FArgs 
       for (int j = 0; j < EPT; ++j) xv[j] = xn[j];
       if (t + 1 < n_units) load_x(u0 + t + 1);
       mbar_wait(&tl.afree[st], sphase ^ 1);     // the MMAs that read this stage have retired
-      if (prod && !(a.dbg & 1)) {
+      if (prod) {
         if (GEN == GEN_UNIFORM) {
           int nan_flag = 0;
 #pragma unroll
@@ -523,7 +521,6 @@ static int launch(const adalog_fused_args* a, cudaStream_t st) {
   k.acc_cols = a->BN <= 64 ? 64 : (a->BN <= 128 ? 128 : 256);
   k.nacc = (int)kTmemCols / k.acc_cols;
   k.epi_warps = a->epi_warps;
-  { const char* e = getenv("ADALOG_B200_FUSED_DBG"); k.dbg = e ? atoi(e) : 0; }   // diagnostics: 1 = no generation, 2 = no epilogue math
   k.brpg = a->brpg; k.g_base = a->g_base; k.u_base = a->u_base;
   k.y = a->y; k.ldy = a->ldy; k.rs = a->rs; k.rs_div = a->rs_div; k.rs_mod = a->rs_mod; k.partial = a->partial;
   const bool i8 = a->dtype == ADALOG_I8;

@@ -14,7 +14,6 @@
 #include "../../include/adalog_b200.h"
 #include <cuda.h>
 #include <cudaTypedefs.h>
-#include <stdlib.h>
 #include <type_traits>
 
 namespace adalog {
@@ -75,8 +74,7 @@ struct KArgs {
 // MODE_PLAIN: yhat = rs*D (attention matmuls)
 // MODE_STORE: no error at all -- out[u*128+p, n] = rs*cs[n]*D + cb[n] is written (the fake-quant INFERENCE forward of a
 // linear layer: rows p of unit u are 128 consecutive tokens, not candidates)
-enum { MODE_CS = 0, MODE_RB = 1, MODE_PLAIN = 2, MODE_NOEPI = 3 /* diagnostic: pipeline only, no epilogue math */,
-       MODE_STORE = 4 };
+enum { MODE_CS = 0, MODE_RB = 1, MODE_PLAIN = 2, MODE_STORE = 4 };
 
 template <int MODE, bool DEBUG, bool I8>
 // 152 registers x 320 threads leave 16.9k registers of the SM free: one 256-thread generator CTA (64 registers) of the
@@ -297,9 +295,7 @@ cand_gemm_err_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_const
           if (c0 + j < ncols) a.dbg[(long long)et * a.N + n0 + c0 + j] = accf(d[j]);
       }
       ocol = c0;
-      if (MODE == MODE_NOEPI) {
-        acc4[0] += __uint_as_float(d[0]);
-      } else if (lim >= 32) {
+      if (lim >= 32) {
 #pragma unroll
         for (int j = 0; j < 32; j += 4) quad(std::false_type{}, d, j, l0, cc, 32, rs, rb);
       } else {
@@ -460,7 +456,6 @@ static int launch(const adalog_gemm_err_args* a, float* dbg, cudaStream_t st, fl
     if (dbg)         ADALOG_LAUNCH_GEMM(MODE_PLAIN, true, false);
     else if (a->cs)  ADALOG_LAUNCH_GEMM(MODE_CS, false, false);
     else if (a->rb)  ADALOG_LAUNCH_GEMM(MODE_RB, false, false);
-    else if (getenv("ADALOG_B200_DIAG_NOEPI")) ADALOG_LAUNCH_GEMM(MODE_NOEPI, false, false);
     else             ADALOG_LAUNCH_GEMM(MODE_PLAIN, false, false);
   }
 #undef ADALOG_LAUNCH_GEMM

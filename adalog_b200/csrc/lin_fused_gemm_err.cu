@@ -33,7 +33,6 @@
 #include "quant_device.cuh"
 #include "../../include/adalog_b200.h"
 #include <algorithm>
-#include <stdlib.h>
 #include <type_traits>
 
 namespace adalog {
@@ -78,7 +77,7 @@ struct LArgs {
   const float* x; long long ldx; int K, U;
   const float* cs; const float* cz; const long long* cq; const float* shift; const float* mtab;
   int P, nl;
-  int KB, N, BN, NT, G, NG, nslot, slotw, SA, SB, streamed, vec, dbg;
+  int KB, N, BN, NT, G, NG, nslot, slotw, SA, SB, streamed, vec;
   const float* y; long long ldy;
   const float* rs; const float* ccs; const float* ccb;
   double* partial;
@@ -165,8 +164,6 @@ lin_fused_kernel(const __grid_constant__ CUtensorMap tmB, const LArgs a) {
   const int u1 = (int)(((long long)(blockIdx.x + 1) * a.U) / gridDim.x);
   const int n_units = u1 - u0;
   const int gen_per_unit = a.streamed ? a.NG : 1;       // how often a unit's A tiles are generated
-  // a wait that spans a whole K loop sleeps between polls; a wait inside the tile pipeline polls
-  const uint32_t nap = a.streamed ? 500u : 100u;
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < kMaxSA; ++i) { mbar_init(&tl.afull[i], kProdWarps); mbar_init(&tl.afree[i], 1); }
@@ -263,12 +260,8 @@ lin_fused_kernel(const __grid_constant__ CUtensorMap tmB, const LArgs a) {
           for (int kb = 0; kb < a.KB; ++kb)
             for (int j = 0; j < a.G; ++j) {
               mbar_wait(&tl.bfree[bs], bph ^ 1);
-              if ((a.dbg & 16) && ((kb + j) & 1)) {            // diagnostic: every other box is not loaded (wrong results)
-                mbar_arrive(&tl.bfull[bs]);
-              } else {
-                mbar_expect_tx(&tl.bfull[bs], bstage);
-                tma_load_2d(&tmB, &tl.bfull[bs], sB + (size_t)bs * bstage, kb * EL, (g * a.G + j) * a.BN);
-              }
+              mbar_expect_tx(&tl.bfull[bs], bstage);
+              tma_load_2d(&tmB, &tl.bfull[bs], sB + (size_t)bs * bstage, kb * EL, (g * a.G + j) * a.BN);
               if (++bs == (uint32_t)a.SB) { bs = 0; bph ^= 1; }
             }
     }
@@ -310,12 +303,10 @@ lin_fused_kernel(const __grid_constant__ CUtensorMap tmB, const LArgs a) {
     }
   } else if (warp == kRelayWarp) {
     // ===================== relay: tfull mbarrier phase -> named-barrier arrival (one polling warp instead of eight) ====
-    if (!(a.dbg & 4)) {
-      const int n_jobs = n_units * a.NT;
-      for (int t = 0; t < n_jobs; ++t) {
-        mbar_wait(&tl.tfull[t & 1], ((uint32_t)t >> 1) & 1);
-        asm volatile("bar.arrive %0, %1;" ::"r"(kBarTile0 + (t & 1)), "n"(kEpiThreads + 32) : "memory");
-      }
+    const int n_jobs = n_units * a.NT;
+    for (int t = 0; t < n_jobs; ++t) {
+      mbar_wait(&tl.tfull[t & 1], ((uint32_t)t >> 1) & 1);
+      asm volatile("bar.arrive %0, %1;" ::"r"(kBarTile0 + (t & 1)), "n"(kEpiThreads + 32) : "memory");
     }
   } else if (warp >= kEpiWarp0 && warp < kTmaWarp) {
     // ===================== epilogue: TMEM -> registers -> per-candidate squared error =====================
@@ -376,18 +367,16 @@ lin_fused_kernel(const __grid_constant__ CUtensorMap tmB, const LArgs a) {
       // "slot ts is full": the relay warp watches the mbarrier and arrives on a named barrier, so that the eight
       // epilogue warps block in hardware instead of polling (ncu, AdaLog fc2 sweep: the nanosleep poll loop of these
       // warps came back every ~45 clocks and was 47% of all executed warp instructions)
-      if (a.dbg & 4) mbar_wait_sleep(&tl.tfull[ts], ((uint32_t)t >> 1) & 1, nap);
-      else asm volatile("bar.sync %0, %1;" ::"r"(kBarTile0 + (int)ts), "n"(kEpiThreads + 32) : "memory");
+      asm volatile("bar.sync %0, %1;" ::"r"(kBarTile0 + (int)ts), "n"(kEpiThreads + 32) : "memory");
       tc_fence_after();
       acc4[0] = acc4[1] = acc4[2] = acc4[3] = 0.0f;
       const uint32_t tbase = tmem_base + lane_base + ts * 256u;
       const int nslab = (ncols + 31) >> 5;
       // this group's 32-column slabs eg, eg+2, ... in 16-column pieces, TMEM -> registers double buffered
       uint32_t da[16], db[16];
-      if (eg < nslab && !(a.dbg & 2)) tmem_ld16(tbase + eg * 32, da);
+      if (eg < nslab) tmem_ld16(tbase + eg * 32, da);
       int l0 = 0;
       for (int sl = eg; sl < nslab; sl += kEpiGroups, l0 += 32) {
-        if (a.dbg & 2) { acc4[0] += 1.0f; break; }    // diagnostic: no TMEM read-out, no error arithmetic
         tmem_ld_wait();
         tmem_ld16(tbase + sl * 32 + 16, db);
         consume(da, l0);
@@ -503,14 +492,11 @@ lin_fused_kernel(const __grid_constant__ CUtensorMap tmB, const LArgs a) {
           asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];"
                        : "=f"(xv[j]), "=f"(xv[j + 1]), "=f"(xv[j + 2]), "=f"(xv[j + 3]) : "r"(xsrc + (uint32_t)j * 32u));
         const float gch = chunk_g[kc / EPT];
-        if (a.dbg & 8) mbar_wait_sleep(&tl.afree[as], aph ^ 1, 200u);
-        else mbar_wait(&tl.afree[as], aph ^ 1);              // the MMAs that read this stage have retired
+        mbar_wait(&tl.afree[as], aph ^ 1);                   // the MMAs that read this stage have retired
         auto store = [&](int i, uint32_t o0, uint32_t o1, uint32_t o2, uint32_t o3) {      // i: compile-time after unrolling
           asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(a_tile + (uint32_t)i * kSoStep), "r"(o0), "r"(o1), "r"(o2), "r"(o3) : "memory");
         };
-        if (a.dbg & 1) {
-          // diagnostic: no generation (pipeline cost only)
-        } else if (!live) {
+        if (!live) {
           // a chunk beyond K (partial last block): the ring stage may hold another block's data from its last use
 #pragma unroll
           for (int i = 0; i < kCPT; ++i) if (i < 2 || has3) store(i, 0u, 0u, 0u, 0u);
@@ -622,11 +608,7 @@ lin_fused_kernel(const __grid_constant__ CUtensorMap tmB, const LArgs a) {
 struct Plan { int KB, BN, NT, G, NG, nslot, slotw, SA, SB, streamed; size_t smem; };
 constexpr size_t kSmemLimit = 227 * 1024 - sizeof(Tail) - 1024;
 
-static int env_int(const char* name, int dflt) { const char* e = getenv(name); return e && *e ? atoi(e) : dflt; }
-
 static int make_plan(const adalog_lin_fused_args* a, Plan* pl) {
-  // tuning overrides (0 = choose): ring depths of the generated (A) and the streamed fixed (B) operand
-  const int want_sa = env_int("ADALOG_B200_LINF_SA", 0), want_sb = env_int("ADALOG_B200_LINF_SB", 0);
   const bool i8 = a->dtype == ADALOG_I8;
   const int EL = i8 ? 128 : 64;
   const bool log = a->gen == ADALOG_GEN_LOG;
@@ -639,12 +621,12 @@ static int make_plan(const adalog_lin_fused_args* a, Plan* pl) {
     const int nt = (a->N + 255) / 256;
     const int BN = std::min(256, std::max(16, r16((a->N + nt - 1) / nt)));
     const size_t bst = (size_t)BN * 128;
-    for (int SB = want_sb ? std::min(want_sb, kMaxSB) : 3; SB >= 2; --SB) {
+    for (int SB = 3; SB >= 2; --SB) {
       const long long room = (long long)kSmemLimit - (long long)lut - (long long)SB * (long long)bst;
       const int SA = (int)std::min<long long>(kMaxSA, room / (long long)kATile);
       if (SA >= pl->KB + 1) {
         pl->BN = BN; pl->NT = (a->N + BN - 1) / BN; pl->G = 1; pl->NG = pl->NT; pl->nslot = 2; pl->slotw = 256;
-        pl->SA = std::min(SA, want_sa ? std::max(want_sa, pl->KB + 1) : 2 * pl->KB); pl->SB = SB; pl->streamed = 0;
+        pl->SA = std::min(SA, 2 * pl->KB); pl->SB = SB; pl->streamed = 0;
         pl->smem = 1024 + (size_t)pl->SA * kATile + (size_t)SB * bst + lut;
         return 0;
       }
@@ -658,10 +640,10 @@ static int make_plan(const adalog_lin_fused_args* a, Plan* pl) {
     const int BN = std::min(256, std::max(16, r16((per_pass + G - 1) / G)));
     const size_t bst = (size_t)BN * 128;
     pl->BN = BN; pl->G = G; pl->NG = passes; pl->NT = passes * G; pl->nslot = 2; pl->slotw = 256; pl->streamed = 1;
-    for (int SB = want_sb ? std::min(want_sb, kMaxSB) : 4; SB >= 2; --SB) {
+    for (int SB = 4; SB >= 2; --SB) {
       const long long room = (long long)kSmemLimit - (long long)lut - (long long)SB * (long long)bst;
-      const int SA = (int)std::min<long long>(want_sa ? want_sa : 6, room / (long long)kATile);
-      if (SA >= (want_sa ? 2 : 3)) {
+      const int SA = (int)std::min<long long>(6, room / (long long)kATile);
+      if (SA >= 3) {
         pl->SA = SA; pl->SB = SB;
         pl->smem = 1024 + (size_t)SA * kATile + (size_t)SB * bst + lut;
         return 0;
@@ -703,7 +685,6 @@ static int launch(const adalog_lin_fused_args* a, cudaStream_t st) {
   k.KB = pl.KB; k.N = a->N; k.BN = pl.BN; k.NT = pl.NT; k.G = pl.G; k.NG = pl.NG; k.nslot = pl.nslot; k.slotw = pl.slotw;
   k.SA = pl.SA; k.SB = pl.SB; k.streamed = pl.streamed;
   k.vec = ((a->ldx & 3) == 0 && (a->K & 3) == 0 && (reinterpret_cast<uintptr_t>(a->x) & 15) == 0) ? 1 : 0;
-  { const char* e = getenv("ADALOG_B200_LINF_DBG"); k.dbg = e ? atoi(e) : 0; }   // diagnostics: 1 = no generation, 2 = no epilogue, 4 = epilogue polls, 8 = producers poll with nanosleep, 16 = half the B loads
   k.y = a->y; k.ldy = a->ldy; k.rs = a->rs; k.ccs = a->ccs; k.ccb = a->ccb; k.partial = a->partial;
   const bool i8 = a->dtype == ADALOG_I8;
   CUtensorMap tmB;

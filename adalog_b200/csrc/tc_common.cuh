@@ -45,30 +45,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     }
   }
 }
-// wait that SLEEPS between polls: for roles that wait long (an epilogue warp while a whole K loop runs).  The plain
-// try_wait loop above is woken by every mbarrier event of the CTA and was measured burning a third of the SM's issue
-// slots in such waits (ncu: 1.3e9 of 4.1e9 warp instructions in one wait loop).
-__device__ __forceinline__ void mbar_wait_sleep(uint64_t* bar, uint32_t parity, uint32_t ns) {
-  const uint32_t addr = smem_u32(bar);
-  uint32_t done = 0;
-  long long t0 = 0;
-  for (uint32_t it = 0;; ++it) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done) : "r"(addr), "r"(parity) : "memory");
-    if (done) break;
-    __nanosleep(ns);
-    if ((it & 0xfff) == 0xfff) {
-      if (t0 == 0) t0 = clock64();
-      else if (clock64() - t0 > 4000000000ll) {
-        printf("adalog: mbarrier timeout (block %d thread %d parity %u)\n", blockIdx.x, threadIdx.x, parity);
-        __trap();
-      }
-    }
-  }
-}
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }

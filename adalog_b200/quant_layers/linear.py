@@ -7,8 +7,6 @@ What differs is underneath: every `_search_best_*` evaluation is one fused devic
 libadalog_b200.so) over HBM-resident calibration tensors instead of a Python loop over 32-sample batches and
 candidate chunks, and the refinement loop is the shared driver in _fpcs.py.
 """
-import os
-
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -24,10 +22,6 @@ __all__ = ['MinMaxQuantLinear', 'PTQSLQuantLinear', 'PTQSLBatchingQuantLinear', 
            'AsymmetricallyChannelWiseBatchingQuantLinear', 'PostGeluTwinUniformBatchingQuantLinear',
            'PostGeluLogBasedBatchingQuantLinear']
 
-# tensor-core inference forward (see PTQSLQuantLinear.quant_forward): opt-in, because the default forward is bit-identical
-# to the reference's F.linear(Q_a(x), Q_w(W), b) and calibration of later layers consumes it; enable per model with
-# utils.wrap_net.set_tensor_core_forward(model, True) or globally with ADALOG_B200_TC_FORWARD=1
-TC_FORWARD = os.environ.get('ADALOG_B200_TC_FORWARD', '0') == '1'
 GELU_MIN = 0.16997124254703522     # -min GELU(x); the post-GELU shift (reference linear.py:749)
 
 
@@ -78,6 +72,11 @@ class MinMaxQuantLinear(nn.Linear):
 class PTQSLQuantLinear(MinMaxQuantLinear):
     """reference: quant_layers/linear.py:64-92 (row-block weight quantisation, n_V sub-matrices)"""
 
+    # tensor-core inference forward (see quant_forward): opt-in, because the default forward is bit-identical to the
+    # reference's F.linear(Q_a(x), Q_w(W), b) and calibration of later layers consumes it; enable per model with
+    # utils.wrap_net.set_tensor_core_forward(model, True)
+    tc_forward = False
+
     def __init__(self, in_features: int, out_features: int, bias: bool = True, mode="raw", w_bit=8, a_bit=8,
                  search_round=1, eq_n=100, n_V=1):
         super().__init__(in_features, out_features, bias=bias, mode=mode, w_bit=w_bit, a_bit=a_bit)
@@ -104,13 +103,12 @@ class PTQSLQuantLinear(MinMaxQuantLinear):
     def quant_forward(self, x):
         """reference linear.py:46-51 with :90-92: F.linear(Q_a(x), Q_w(W), b), bit-identical to the reference's
         composition (the quantizers are the sm_100a kernels, the product is FP32).  With `tc_forward` enabled
-        (set_tensor_core_forward / ADALOG_B200_TC_FORWARD=1; inference only: no grad, no training_mode) the same
-        product is ONE exact integer GEMM on the tensor cores with the dequantisation in its epilogue
+        (set_tensor_core_forward; inference only: no grad, no training_mode) the same product is ONE exact integer
+        GEMM on the tensor cores with the dequantisation in its epilogue
         (sweep.linear_quant_forward; weight operand cached until the weight or its quantizer changes): equal to the
         FP32 composition to FP32 rounding (<= 2e-5 of the output range, tests/test_gpu_gemm.py), not bit for bit."""
         assert self.calibrated, f"Module should be calibrated before run quant_forward for {self}"
-        tc = self.__dict__.get('tc_forward')
-        if ((TC_FORWARD if tc is None else tc) and x.is_cuda and x.dtype == torch.float32 and not torch.is_grad_enabled()
+        if (self.tc_forward and x.is_cuda and x.dtype == torch.float32 and not torch.is_grad_enabled()
                 and not self.w_quantizer.training_mode and not self.a_quantizer.training_mode
                 and self.w_quantizer.n_bits < 32 and self.a_quantizer.n_bits < 32):
             cache = self.__dict__.setdefault('_tc_cache', {})

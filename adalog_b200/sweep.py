@@ -11,7 +11,6 @@ and the scales, biases and shift corrections are applied in the fused epilogue.
 """
 import functools
 import math
-import os
 
 import torch
 
@@ -21,15 +20,9 @@ from .utils import dist as adist
 
 # operand workspace of the generator -> GEMM path (two buffers of half this size).  8 GiB of the 180 GB: fewer, larger
 # chunks -- the DeiT-B fc2 AdaLog sweep (9.9 GB of candidate operand) measured 16.1 ms with 2 GiB, 14.7 ms with 8 GiB
-WS_BYTES = int(os.environ.get('ADALOG_B200_WS_MB', '8192')) << 20
+WS_BYTES = 8 << 30
 NUM_SMS = 148
 R_BASE = 37.0
-# uniform x uniform sweeps (every quantizer up to 7 bits: |code - zp| <= 127) run on the INT8 tensor cores
-# (tcgen05.mma.kind::i8, S32 accumulation: exact) at twice the bf16 MMA rate and half the operand bytes
-USE_I8 = os.environ.get('ADALOG_B200_I8', '1') == '1'
-
-# linear activation sweeps: generate the candidate operand inside the GEMM kernel (0: generator -> workspace -> GEMM)
-LIN_FUSED = os.environ.get('ADALOG_B200_LIN_FUSED', '1') != '0'
 
 
 def _lin_fused_passes():
@@ -38,12 +31,8 @@ def _lin_fused_passes():
     (tests/gpu_lin_bench.py, fused vs two-kernel, ms per evaluation): DeiT-S int8 K=384: N=1152 1.78 vs 2.15, N=384 1.10
     vs 1.16, N=1536 2.05 vs 2.36, AdaLog K=1536 N=384 4.08 vs 5.41; DeiT-B int8 K=768: N=2304 4.31 vs 4.93, N=768 2.09
     vs 2.40, N=3072 5.51 vs 6.47.  Only the schedules that regenerate the operand (DeiT-B AdaLog K=3072 N=768: two
-    512-column TMEM passes, 17.4 vs 16.9) stay on the two-kernel path.  ADALOG_B200_LIN_FUSED=force takes the fused
-    kernel wherever it fits, =0 never."""
-    mode = os.environ.get('ADALOG_B200_LIN_FUSED', '1')
-    if not LIN_FUSED or mode == '0':
-        return None
-    return 1 << 30 if mode == 'force' else 1
+    512-column TMEM passes, 17.4 vs 16.9) stay on the two-kernel path."""
+    return 1
 
 _workspaces = {}
 
@@ -76,7 +65,6 @@ def _pad128(t, dim=-1):
     return t.index_select(dim, idx)
 
 
-OVERLAP = os.environ.get('ADALOG_B200_OVERLAP', '1') == '1'
 _side = {}
 
 
@@ -155,7 +143,7 @@ def run_cand_gemm(gen_cand, U, ka, UG, Bm, brpg, N, y, ldy, rs, rb=None, rs_div=
     n_chunks = (U + step - 1) // step
     BN = ops.pick_bn(N, 32 if rb is not None else 16)
     NT = (N + BN - 1) // BN
-    overlap = OVERLAP and n_chunks > 1 and dev.type == 'cuda'
+    overlap = n_chunks > 1 and dev.type == 'cuda'
     ws_all = _workspace(dev, (2 if overlap else 1) * step * unit_elems)
     bufs = [ws_all[:step * unit_elems], ws_all[step * unit_elems:]] if overlap else [ws_all]
 
@@ -263,10 +251,12 @@ def linear_err_a_self(ctx, cs, cz, n_levels, channel_wise):
 
 
 def _i8_ok(*n_levels):
-    return USE_I8 and all(nl <= 64 for nl in n_levels)
+    """uniform x uniform sweeps (every quantizer up to 7 bits: |code - zp| <= 127) run on the INT8 tensor cores
+    (tcgen05.mma.kind::i8, S32 accumulation: exact) at twice the bf16 MMA rate and half the operand bytes"""
+    return all(nl <= 64 for nl in n_levels)
 
 
-FIXED_CACHE = os.environ.get('ADALOG_B200_FIXED_CACHE', '1') == '1'
+FIXED_CACHE = True     # False rebuilds the fixed operand on every evaluation: the reference the cache is tested against
 
 
 def _pkey(*tensors):
@@ -446,10 +436,11 @@ def linear_err_a(ctx, weight3, bias, wq, cs, cz, n_levels_a, y2d=None):
     ntok = ctx.x2d.shape[0]
     y = ctx.y2d if y2d is None else y2d
     res = None
-    if out_f % 4 == 0 and _lin_fused_passes() is not None:
+    passes = _lin_fused_passes()
+    if out_f % 4 == 0 and passes is not None:
         # candidates generated inside the GEMM kernel: one launch, nothing expanded in HBM (lin_fused_gemm_err.cu)
         res = ops.lin_fused_cand_gemm_err(ctx.x2d, Bm, out_f, y, rs, s_w.contiguous(), cb.contiguous(), n_levels_a, P,
-                                          c1, cz=z1, i8=i8, max_passes=_lin_fused_passes())
+                                          c1, cz=z1, i8=i8, max_passes=passes)
     if res is None:
         res = run_cand_gemm(gen, ntok, ka, ntok, Bm, 0, out_f, y, out_f, rs, None, 1 << 62, 1, s_w, cb,
                             k_true=in_f, i8=i8)
@@ -499,9 +490,10 @@ def linear_err_log(ctx, weight3, bias, wq, aq, cs, cq):
     cb = (b - shift.double() * s_w.double() * colsum.double()).float().contiguous()
     ntok = ctx.x2d.shape[0]
     res = None
-    if out_f % 4 == 0 and _lin_fused_passes() is not None:
+    passes = _lin_fused_passes()
+    if out_f % 4 == 0 and passes is not None:
         res = ops.lin_fused_cand_gemm_err(ctx.x2d, Bm, out_f, ctx.y2d, rs, s_w.contiguous(), cb, nl, P, c1, cq=q1,
-                                          shift=shift, mtab=mtab, max_passes=_lin_fused_passes())
+                                          shift=shift, mtab=mtab, max_passes=passes)
     if res is None:
         res = run_cand_gemm(gen, ntok, ka, ntok, Bm, 0, out_f, ctx.y2d, out_f, rs, None, 1 << 62, 1, s_w, cb,
                             k_true=in_f)
@@ -549,7 +541,8 @@ def _matmul_reduce(res, ctx, P, head_channel_wise, pool_heads, n_cols_total):
     return (tot[:P] / -((n_cols_total * ctx.H))).float()                    # [P]
 
 
-FUSED = os.environ.get('ADALOG_B200_FUSED', '1') == '1'
+# False sends every attention sweep through generator -> workspace -> GEMM: the path the fused kernel is tested against
+FUSED = True
 
 
 @functools.lru_cache(maxsize=1024)
@@ -571,9 +564,7 @@ def _use_fused(K, N, i8, log, n_levels):
     """The fused generator + GEMM kernel is taken where it measured faster than generator -> workspace -> GEMM
     (DeiT-S, 128 images: QK^T sweeps 1.95 vs 2.44 ms, P.V base search 5.3 vs 5.8 ms); for a uniform candidate side with
     a long reduction (P.V value sweep, K = 197) its 14 worker warps are short of issue slots (2.3 vs 1.9 ms)."""
-    if not FUSED or ops.fused_plan(K, N, i8, log, n_levels) is None:
-        return False
-    return log or K <= 128 or os.environ.get('ADALOG_B200_FUSED_LONGK', '0') == '1'
+    return FUSED and ops.fused_plan(K, N, i8, log, n_levels) is not None and (log or K <= 128)
 
 
 def _run_fused(x2d, K, Bm, N, U, UG, y, ldy, rs, H, n_levels, P, i8=False, **cand):

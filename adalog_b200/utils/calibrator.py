@@ -5,7 +5,6 @@ hyperparameter_searching(), reparam() where a preceding LayerNorm is attached, f
 'quant_forward' -- but the captured tensors stay in HBM (no .cpu() round trip per batch, reference :14-28) where the
 device sweeps consume them directly.  Under torch.distributed each rank captures its own shard of the loader.
 """
-import os
 import time
 
 import torch
@@ -24,9 +23,9 @@ class QuantCalibrator:
         self.model = model
         self.calib_loader = calib_loader
         self.progress = True
-        # ADALOG_B200_TIMING=1: synchronise around capture / search of every module and keep the seconds in
+        # timing (set by the caller): synchronise around capture / search of every module and keep the seconds in
         # self.timings[name] = (capture_s, search_s) -- for profiling only (adds two device syncs per module)
-        self.timing = os.environ.get('ADALOG_B200_TIMING', '0') == '1'
+        self.timing = False
         self.timings = {}
         # Block-resume capture (SURVEY.md section 8f rank 1): the reference re-runs the WHOLE model over the
         # calibration set for every module (74 full forwards for a ViT).  A module inside a transformer block only
@@ -34,7 +33,6 @@ class QuantCalibrator:
         # (reparam rewrites the block's LayerNorm/linear, i.e. what comes after the input).  So the input of each
         # block is captured once with one full forward and the block alone is replayed per module: same kernels on
         # the same tensors, hence bit-identical captures, at 1/4 of the forward work.
-        self.fast_capture = os.environ.get('ADALOG_B200_FAST_CAPTURE', '1') == '1'
         self.block_types = (_zoo.Block, _zoo.SwinTransformerBlock)
         self._cached_block = None
         self._cached_inputs = None
@@ -87,7 +85,7 @@ class QuantCalibrator:
                 and isinstance(self._by_name.get(pp), torch.nn.Sequential))
 
     def _run_forwards(self, name, device):
-        block = self._enclosing_block(name) if self.fast_capture else None
+        block = self._enclosing_block(name)
         with torch.no_grad():
             if block is None:
                 self._cached_block = self._cached_inputs = None

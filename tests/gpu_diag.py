@@ -110,7 +110,7 @@ def perf_probe():
                 fl, ms, n = ops.profile_gemm_summary()
                 ops.profile_reset(False)
                 print(f'   {nm}: {t:.2f} ms; GEMM kernel {ms / 3:.2f} ms in {n // 3} launches ({fl / ms / 1e9:.0f} TFLOP/s); '
-                      f'rest {t - ms / 3:.2f} ms  [overlap={sweep.OVERLAP}]')
+                      f'rest {t - ms / 3:.2f} ms')
 
 
 def perf_matmul():

@@ -72,11 +72,12 @@ def main():
             print(f'{which} {name:5s} K={in_f:5d} N(tokens)={tokens} units={out_f:5d} W-side {"bf16" if log else "i8"}: '
                   f'{t_w:7.3f} ms ({2.0 * 128 * tokens * in_f * out_f / t_w / 1e9:7.0f} Tops/s)', flush=True)
             continue
-        os.environ['ADALOG_B200_LIN_FUSED'] = 'force'
+        policy = sweep._lin_fused_passes
+        sweep._lin_fused_passes = lambda: 1 << 30      # fused wherever it fits
         t_f = timeit(fn)
-        os.environ['ADALOG_B200_LIN_FUSED'] = '0'
+        sweep._lin_fused_passes = lambda: None         # two-kernel path
         t_p = timeit(fn)
-        os.environ.pop('ADALOG_B200_LIN_FUSED')
+        sweep._lin_fused_passes = policy
         ops = 2.0 * 128 * tokens * in_f * out_f
         print(f'{which} {name:5s} K={in_f:5d} N={out_f:5d} {"log bf16" if log else "uniform i8"}: fused {t_f:7.3f} ms '
               f'({ops / t_f / 1e9:7.0f} Tops/s)   two-kernel {t_p:7.3f} ms ({ops / t_p / 1e9:7.0f} Tops/s)', flush=True)

@@ -1,5 +1,5 @@
 """ncu target (not a pytest file): the AdaLog activation sweep and the weight sweep of a DeiT-B fc2-shaped layer
-(128 images x 197 tokens, K=3072, N=768), OVERLAP off so each kernel is profiled alone.
+(128 images x 197 tokens, K=3072, N=768).
   ncu --set full --clock-control none --import-source on -k regex:'gen_log_cand|cand_gemm_err' -c 6 python tests/gpu_ncu_fc2.py"""
 import os
 import sys
@@ -9,7 +9,6 @@ import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'oracle'))
-os.environ.setdefault('ADALOG_B200_OVERLAP', '0')
 from adalog_b200 import sweep  # noqa: E402
 from adalog_b200.quantizers import ShiftAdaLogQuantizer, UniformQuantizer  # noqa: E402
 import adalog_oracle as O  # noqa: E402  (candidate seeding only; this is a profiling helper, not product code)

@@ -8,7 +8,6 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-os.environ['ADALOG_B200_TIMING'] = '1'
 import bench  # noqa: E402
 from adalog_b200.utils.calibrator import QuantCalibrator  # noqa: E402
 
@@ -22,6 +21,7 @@ for rep in range(2):
     loader = [(images[i:i + 32], None) for i in range(0, n_img, 32)]
     cal = QuantCalibrator(model, loader)
     cal.progress = False
+    cal.timing = True
     torch.cuda.synchronize()
     t0 = time.perf_counter()
     cal.batching_quant_calib()

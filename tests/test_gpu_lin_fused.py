@@ -29,18 +29,12 @@ def _setup(tokens, in_f, out_f, gelu=False, seed=3):
 
 
 def _both(fn):
-    import os
-    old = os.environ.get('ADALOG_B200_LIN_FUSED')
-    try:
-        os.environ['ADALOG_B200_LIN_FUSED'] = 'force'      # every shape that fits, not only the ones the heuristic picks
+    from adalog_b200 import sweep
+    with pytest.MonkeyPatch.context() as mp:
+        mp.setattr(sweep, '_lin_fused_passes', lambda: 1 << 30)   # every shape that fits, not only the ones the policy picks
         fused = fn()
-        os.environ['ADALOG_B200_LIN_FUSED'] = '0'
+        mp.setattr(sweep, '_lin_fused_passes', lambda: None)
         plain = fn()
-    finally:
-        if old is None:
-            os.environ.pop('ADALOG_B200_LIN_FUSED', None)
-        else:
-            os.environ['ADALOG_B200_LIN_FUSED'] = old
     return fused, plain
 
 
@@ -54,7 +48,7 @@ def _both(fn):
     (2000, 192, 192, 8),       # 8-bit activations: bf16 uniform operands
     (900, 768, 768, 8),        # bf16 uniform, 12 K blocks: STREAMED, 2 passes
 ])
-def test_uniform_sweep_matches_two_kernel_path(tokens, in_f, out_f, bits):
+def test_fused_uniform_sweep_matches_two_kernel_path(tokens, in_f, out_f, bits):
     from adalog_b200 import ops, sweep
     nl = 2 ** (bits - 1)
     x, W, b, y = _setup(tokens, in_f, out_f)
@@ -93,7 +87,7 @@ def test_uniform_sweep_matches_two_kernel_path(tokens, in_f, out_f, bits):
     (700, 200, 52, 6),         # ragged K, 6-bit LUT
     (100, 512, 128, 4),        # fewer units than SMs
 ])
-def test_log_sweep_matches_two_kernel_path(tokens, in_f, out_f, bits):
+def test_fused_log_sweep_matches_two_kernel_path(tokens, in_f, out_f, bits):
     from adalog_b200 import ops, sweep
     from adalog_b200.quantizers import ShiftAdaLogQuantizer
     nl = 2 ** (bits - 1)
